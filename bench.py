@@ -14,6 +14,16 @@ generation:
 
     python bench.py [--gpus N] [--steps K] [--warmup W]              our CUDA path (one JSON line on rank 0)
     python bench.py --impl reference ...                            the CPU reference arm (oracle port, all host threads)
+    python bench.py --dump-outputs DIR ...                          also write what the timed path returned as DIR/<name>.npy
+
+--steps K times exactly K decode steps after the warm-up, or is refused when one generation cannot hold them; the edit
+workload times whole sessions, whose length the workload sets, and takes no --steps.
+--dump-outputs: inputs, weights and random streams are fixed by seeds, so two builds run with the same arguments can be
+compared output for output.  tts: `tokens` [B, steps so far, K] (every utterance's delayed token rows up to and including
+the last timed step) and `logits` [B, K, V] (the logits that step sampled from).  edit: `tokens` [N, K, T'max] (each
+edited token matrix, padded with -1) and `lengths` [N].  float32 (token ids are exact), at most 64 MB (beyond that, a
+fixed seeded sample of the utterances, their indices in `utterances`); with N > 1 GPUs every rank writes its own
+utterances, the names suffixed with _rank<r>.  DIR = bench_outputs/ inside the tree is ignored by git.
 
 value    = whole-job codec tokens/s, device-timed (CUDA events on the launching stream, max over ranks), inputs resident
            in HBM.  tts: K timed steps form a window CENTRED on the mean context of the 16 s generation (ctx 231 -> 881,
@@ -35,14 +45,18 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
+
+DUMP_LIMIT = 64 << 20
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=600)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed decode steps, exactly (600; reference arm: 64); the edit workload times whole sessions")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed decode steps before them (10; reference arm: 2)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="tts", choices=["tts", "edit"])
     ap.add_argument("--model", default="830M")
@@ -55,7 +69,19 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-repeats", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    if a.impl == "ours" and a.workload == "edit" and a.steps is not None:
+        ap.error("--steps: the edit workload times whole editing sessions, whose length the workload sets")
+    if a.steps is None:
+        a.steps = 64 if a.impl == "reference" else 600
+    if a.warmup is None:
+        a.warmup = 2 if a.impl == "reference" else 10
+    if a.warmup < 0:
+        ap.error("--warmup must be >= 0")
     if a.batch is None:
         a.batch = 32 if a.workload == "tts" else 16
     if a.text_len is None:
@@ -179,9 +205,26 @@ def host_threads():
     return int(env) if env else max(1, min(n, 64))
 
 
-def cpu_baseline(args, cfg, sd, utts, steps, threads=None):
+def decode_steps(args, cfg):
+    """decode steps of one utterance until the reference's length cap (y_len > x_len * encodec_sr / 5) ends it"""
+    return args.text_len * (cfg.encodec_sr // 5) - (args.prompt + 1) - 2
+
+
+def check_steps(args):
+    """--steps is exactly the number of timed decode steps: refuse, before any work, a count one generation cannot hold
+    after the warm-up (the CUDA arm also keeps a few steps after the window for its profiled pass)."""
+    from voicecraft_b200 import synthetic
+    W = args.warmup if args.impl == "reference" else max(3, args.warmup)
+    top = decode_steps(args, synthetic.make_config(args.model)) - W - 10
+    if not 1 <= args.steps <= top:
+        raise SystemExit(f"--steps {args.steps}: a --text-len {args.text_len}, --prompt {args.prompt} generation holds 1 to "
+                         f"{top} timed steps after {W} warm-up steps")
+
+
+def cpu_baseline(args, cfg, sd, utts, steps, threads=None, warm=0):
     """The oracle port of the reference's own batched decode (inference_tts_batch, B copies of one prompt ==
-    the compute of B independent utterances of that length) timed on the host cores, bounded sample."""
+    the compute of B independent utterances of that length) timed on the host cores, bounded sample: `steps` decode
+    steps after `warm` untimed ones."""
     from oracle import lm_oracle
     threads = threads or host_threads()
     torch.set_num_threads(threads)
@@ -191,13 +234,14 @@ def cpu_baseline(args, cfg, sd, utts, steps, threads=None):
     torch.manual_seed(1)
     B = 32 if args.workload == "tts" else args.batch
     oracle.inference_tts_batch(x, x_lens, y, top_k=40, top_p=1.0, temperature=1.0, stop_repetition=3,
-                               batch_size=B, max_steps=steps + 1, on_step=lambda c: marks.append(time.perf_counter()))
-    dt = marks[-1] - marks[0]                      # decode steps only (the first mark is after prefill + first sample)
-    n = len(marks) - 1
+                               batch_size=B, max_steps=warm + steps + 1, on_step=lambda c: marks.append(time.perf_counter()))
+    dt = marks[-1] - marks[warm]                   # decode steps only (the first mark is after prefill + first sample)
+    n = len(marks) - 1 - warm
+    assert n == steps, (n, steps)
     tok_s = B * cfg.n_codebooks * n / dt
     return dict(value=tok_s, unit="codec tokens/s", cores=threads, kind="port",
                 sample=f"oracle inference_tts_batch B={B}, {n} decode steps after a {args.text_len + args.prompt + 1}-token "
-                       f"prefill, fp32, {threads} threads, {dt / n * 1e3:.0f} ms/step"), dt / n
+                       f"prefill and {warm} warm-up steps, fp32, {threads} threads, {dt / n * 1e3:.0f} ms/step"), dt / n
 
 
 def workload_config(args, cfg, world=1):
@@ -223,15 +267,30 @@ def run_reference(args):
         return
     cfg, sd = make_model(args)
     utts = make_utterances(args, cfg, range(1))
-    steps = max(1, min(args.steps, 64))
-    warm = max(0, min(args.warmup, 2))
-    cb, ms = cpu_baseline(args, cfg, sd, utts, steps + warm)
+    steps, warm = args.steps, args.warmup
+    cb, ms = cpu_baseline(args, cfg, sd, utts, steps, warm=warm)
     line = {"impl": "reference", "metric": "codec tokens/s (830M TTS decode)", "value": cb["value"], "unit": "codec tokens/s",
             "n_gpus": args.gpus, "steps": steps, "warmup": warm, "ms_per_step": ms * 1e3, "higher_is_better": True,
             "scaling": "weak" if args.workload == "tts" else "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": workload_config(args, cfg, args.gpus), "cpu_baseline": cb,
             "e2e": {"value": cb["value"], "unit": "codec tokens/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
+
+
+def dump_outputs(path, arrays, rank, world):
+    """--dump-outputs: one float32 DIR/<name>.npy per array (see the module docstring).  Every array is indexed by utterance
+    first; above DUMP_LIMIT bytes in all, a fixed seeded sample of the utterances is written, their indices in `utterances`."""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(n, size=max(1, n * DUMP_LIMIT // total - 1), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["utterances"] = keep.astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + suffix + ".npy"), a)
 
 
 def traffic_record(kernel_name):
@@ -319,9 +378,9 @@ def run_tts(args, D):
     model.load_state_dict(sd)
     model = model.to(dev).eval()
     cap = args.text_len * (cfg.encodec_sr // 5)
-    S_total = cap - (args.prompt + 1) - 2                  # decode steps until the length cap fires
+    S_total = decode_steps(args, cfg)
     W = max(3, args.warmup)
-    Ksteps = max(1, min(args.steps, S_total - W - 10))
+    Ksteps = args.steps                                    # in range: check_steps()
     start = max(W, (S_total - Ksteps) // 2)                # window centred on the mean context of the generation
     model.configure_engine(max_slots=B, max_seq_len=(args.text_len + cap + 64 + 255) // 256 * 256, kv_dtype=args.kv,
                            max_new_tokens=cap + 64)
@@ -353,6 +412,11 @@ def run_tts(args, D):
     st = sess.poll()
     assert all(s.n_steps == 1 + start + Ksteps for s in st), [s.n_steps for s in st]
     assert not any(s.done for s in st)
+    if args.dump_outputs:
+        logits = torch.empty(B * K, sess.V, device=dev)
+        _lib.check(lib.vcb_debug_logits(eng, logits.data_ptr(), B * K))
+        dump_outputs(args.dump_outputs, {"tokens": np.stack([sess.raw_tokens(i) for i in range(B)]),
+                                         "logits": logits.view(B, K, sess.V).cpu()}, rank, world)
     tok_s = world * B * K * Ksteps / (ms * 1e-3)
     ctx1 = ctx0 + Ksteps
 
@@ -485,6 +549,12 @@ def run_edit(args, D):
     # generated frames replace the 100-frame span: T' = T - 100 + generated
     gen_frames_total = D.sum(sum(int(r.shape[-1]) - (args.prompt - 100) for r in res))
     tok_s = gen_frames_total * K / (ms * 1e-3)
+    if args.dump_outputs:
+        lengths = [int(r.shape[-1]) for r in res]
+        tokens = torch.full((len(res), K, max(lengths, default=0)), -1, dtype=torch.int64)
+        for i, r in enumerate(res):
+            tokens[i, :, : lengths[i]] = r[0].cpu()
+        dump_outputs(args.dump_outputs, {"tokens": tokens, "lengths": lengths}, rank, world)
 
     # ---- e2e: host in -> inference_many -> NCCL gather -> host out
     times, comm, full = [], 0, None
@@ -522,6 +592,8 @@ def run_edit(args, D):
 
 def main():
     args = parse()
+    if args.impl == "reference" or args.workload == "tts":
+        check_steps(args)
     if args.impl == "reference":
         return run_reference(args)
     D = Dist()

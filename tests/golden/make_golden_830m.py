@@ -31,6 +31,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.dirname(HERE))
+
+import golden_util  # noqa: E402
 
 N_STEPS = 64
 PROMPTS = [150, 170, 400, 420, 230, 330, 110, 460]       # ctx = 80 + p + 1: 231, 251, 481, 501, 311, 411, 191, 541
@@ -156,6 +159,7 @@ def part_b(out, t0):
         out[f"logits_{pol}"] = np.stack([traces[i] for i in TRACE_UTTS]).astype(np.float32)   # [utt, step, K, V]
         del oracle
     lm_oracle.sample_rows = orig
+    out["logits_bf16_planes"] = golden_util.pack_logits_delta(out["logits_fp32"], out.pop("logits_bf16"))
     np.savez_compressed(os.path.join(HERE, "lm_830m_b32.npz"), **out)
     meta = dict(n_steps=N_STEPS, prompts=PROMPTS, text_len=TEXT_LEN, kw=KW, trace_utts=TRACE_UTTS, trace_steps=TRACE_STEPS,
                 pinned=pinned, pinned_ckpt_seed=3, ckpt_seed=0, noise_seed="1 + i", data_seed="100 + i")
